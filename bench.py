@@ -6,8 +6,9 @@ Mnih'15 Q-network, Huber loss, centered RMSProp (examples/dqn/mnih15 config), ga
 target update every 2500 steps.  One "step" = get_next(256, 2) + DqnAgent.train(experience).
 
   value        steps/s with the ring resident in HBM; the step is replayed as ONE CUDA graph.
-               `--steps K` steps are timed `--repeats R` times (each block bracketed by
-               barrier + synchronize, CUDA events, max over ranks); value is the MEDIAN block.
+               `--steps K` steps are timed `--repeats R` times (default once; each block
+               bracketed by barrier + synchronize, CUDA events, max over ranks); value is the
+               MEDIAN block.  The e2e arm and the update-only roofline also time K steps.
   e2e          the same step through the public API with HOST buffers: every step copies one
                driver step of collected frames (256 x 28 244 B) from pinned host memory,
                add_batch, get_next, train, and reads that step's loss back (the read of step
@@ -25,7 +26,13 @@ target update every 2500 steps.  One "step" = get_next(256, 2) + DqnAgent.train(
 The main line is complete before the extra configs and the CPU arm start; they only add keys, and
 a watchdog (`--extras-timeout`, 600 s) prints the line without them should one of them hang.
 
-`--impl reference` times that CPU restatement alone (the reference arm of the contract).
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step computed as
+DIR/<name>.npy (float32 / float64): its loss, td_loss and td_error, the Q-network and target-network
+parameters after the update, and the batch it trained on (ids, probabilities, the scalar leaves and
+a fixed seeded sample of the observation bytes).  Every input is seeded, so two builds run with the
+same arguments can be compared output for output.
+
+`--impl reference` times that CPU restatement alone (the reference arm of the project).
 N>1 (torchrun): one process per GPU, each with its own 1M-slot ring shard and a local batch of
 256; gradients are SUM-all-reduced (NCCL) every step, loss is divided by the global batch
 (utils/common.py:1465-1467).  value = batch-256-equivalent train steps/s of the whole job
@@ -243,8 +250,8 @@ def run_reference(args):
   rank = int(os.environ.get('RANK', '0'))
   if rank != 0:
     return
-  steps = max(1, min(args.steps, 20))
-  warm = max(3, min(args.warmup, 5))
+  steps = args.steps
+  warm = max(3, args.warmup)
   arm = CpuArm()
   sps, sweep, sample = arm.measure(steps, warm)
   line = dict(
@@ -275,12 +282,39 @@ def _oracle_layers(net, Ly):
   return layers
 
 
+OBS_SAMPLE = 1 << 16        # observation bytes of the trained batch written by --dump-outputs
+
+
+def dump_outputs(out_dir, loss_info, batch, net, target_net):
+  """Writes the last timed step's results as out_dir/<name>.npy (float32, or float64 for the
+  int64 ids and the integer leaves so that they stay exact)."""
+  exp, info = batch
+  tensors = dict(loss=loss_info.loss, td_loss=loss_info.extra.td_loss,
+                 td_error=loss_info.extra.td_error, q_network_params=net.flat_params,
+                 target_q_network_params=target_net.flat_params, ids=info.ids,
+                 probabilities=info.probabilities)
+  for name in ('step_type', 'action', 'next_step_type', 'reward', 'discount'):
+    tensors[name] = getattr(exp, name)
+  arrays = {k: t.detach().cpu().numpy() for k, t in tensors.items()}
+  obs = exp.observation.cpu().numpy().reshape(-1)
+  pick = np.sort(np.random.RandomState(0).choice(obs.size, min(OBS_SAMPLE, obs.size), replace=False))
+  arrays['observation_sample'] = obs[pick]
+  arrays = {k: a.astype(np.float32 if a.dtype in (np.float32, np.uint8) else np.float64)
+            for k, a in arrays.items()}
+  total = sum(a.nbytes for a in arrays.values())
+  assert total <= 64 << 20, f'--dump-outputs would write {total} bytes'
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--gpus', type=int, default=1)
-  ap.add_argument('--steps', type=int, default=200)
+  ap.add_argument('--steps', type=int, default=200, help='train steps in each timed loop')
   ap.add_argument('--warmup', type=int, default=10)
-  ap.add_argument('--repeats', type=int, default=9)
+  ap.add_argument('--repeats', type=int, default=1,
+                  help='timed blocks of --steps steps for `value` (its median block)')
   ap.add_argument('--impl', default='b200')
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--no-graph', action='store_true')
@@ -293,7 +327,11 @@ def main():
   ap.add_argument('--ncu-step', action='store_true',
                   help='after warm-up run ONE un-captured step between cudaProfilerStart/Stop and '
                        'exit (target of `ncu --profile-from-start off`; prints no bench value)')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='write what the last timed step computed to DIR/<name>.npy')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be >= 1')
   if args.impl == 'reference':
     return run_reference(args)
 
@@ -403,7 +441,8 @@ def main():
   # (agents/dqn/examples/v2/train_eval.py:226-232): the next batch is produced while the current
   # one trains.  Here: two sample buffers; step i trains on buffer i & 1 while the sampler fills
   # the other one on a side stream (same Philox draw order as back-to-back calls).  Every step
-  # still contains one sample and one train.
+  # still contains one sample and one train.  A step returns (LossInfo, the (experience,
+  # BufferInfo) batch it trained on).
   prefetch = not args.no_prefetch
   side_stream = torch.cuda.Stream(device=dev)
   sample_bufs = [rb.get_next(sample_batch_size=B, num_steps=T) for _ in range(2)]
@@ -415,14 +454,14 @@ def main():
       side_stream.wait_stream(main)
       with torch.cuda.stream(side_stream):
         rb.get_next(sample_batch_size=B, num_steps=T, out=sample_bufs[slot ^ 1])
-      loss_ = agent.train(sample_bufs[slot][0]).loss
+      loss_info = agent.train(sample_bufs[slot][0])
       main.wait_stream(side_stream)
-      return loss_
+      return loss_info, sample_bufs[slot]
     return body
 
   def serial_step():
-    exp, _ = rb.get_next(sample_batch_size=B, num_steps=T)
-    return agent.train(exp).loss
+    batch = rb.get_next(sample_batch_size=B, num_steps=T)
+    return agent.train(batch[0]), batch
 
   bodies = [pipelined(0), pipelined(1)]
 
@@ -498,7 +537,7 @@ def main():
     sync_all()
     e0.record()
     for _ in range(K):
-      loss = fn()
+      loss_info, batch = fn()
     e1.record()
     sync_all()
     ms = e0.elapsed_time(e1)
@@ -507,6 +546,10 @@ def main():
       dist.all_reduce(t, op=dist.ReduceOp.MAX)
       ms = float(t.item())
     block_ms.append(ms)
+  # graph outputs are overwritten by the next replay: read the last timed step's results now
+  final_loss = float(loss_info.loss.item())
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, loss_info, batch, net, agent._target_q_network)
   # keep the sampler running over a load of at least ~1.5 s so that it sees the step's clocks
   while time.perf_counter() - t_wall0 < 1.5:
     for _ in range(K):
@@ -514,7 +557,6 @@ def main():
     torch.cuda.synchronize()
   clk = clocks.stop()
   ms = float(np.median(block_ms))
-  final_loss = float(loss.item())
   agent.check_numerics()
   steps_per_s = K / (ms / 1000.0)
   value = steps_per_s * world                  # batch-256-equivalent steps/s of the whole job
@@ -542,7 +584,7 @@ def main():
   gather_ms = ge0.elapsed_time(ge1) / (n_g * reps)
   del outs, gg
   exp, _ = rb.get_next(sample_batch_size=B, num_steps=T)
-  n_u = max(10, min(K, 50))
+  n_u = K
   ue0, ue1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
   # the update alone, replayed from its own graph so that the events bracket GPU time
   train_only = common.function(lambda: agent.train(exp), warmup=1) if use_graph else (
@@ -564,12 +606,13 @@ def main():
   update_tfs = FLOPS_PER_STEP / (update_ms * 1e-3) / 1e12
 
   # ---- e2e: host buffers in, loss out, every step -----------------------------------------------
-  Ke = max(10, min(K, 200))
-  host = [torch.randint(0, 3, (B_ENV,), dtype=torch.int32).pin_memory(),
-          torch.randint(0, 256, (B_ENV, 84, 84, 4), dtype=torch.uint8).pin_memory(),
-          torch.randint(0, A, (B_ENV,), dtype=torch.int32).pin_memory(),
-          torch.randint(0, 3, (B_ENV,), dtype=torch.int32).pin_memory(),
-          torch.rand(B_ENV).pin_memory(), torch.ones(B_ENV).pin_memory()]
+  Ke = K
+  gh = torch.Generator().manual_seed(4321 + rank)
+  host = [torch.randint(0, 3, (B_ENV,), dtype=torch.int32, generator=gh).pin_memory(),
+          torch.randint(0, 256, (B_ENV, 84, 84, 4), dtype=torch.uint8, generator=gh).pin_memory(),
+          torch.randint(0, A, (B_ENV,), dtype=torch.int32, generator=gh).pin_memory(),
+          torch.randint(0, 3, (B_ENV,), dtype=torch.int32, generator=gh).pin_memory(),
+          torch.rand(B_ENV, generator=gh).pin_memory(), torch.ones(B_ENV).pin_memory()]
   h2d = sum(t.numel() * t.element_size() for t in host)
 
   # Double-buffered upload: the pinned->device copy of step i+1's frames runs on a copy stream
@@ -608,7 +651,7 @@ def main():
       consumed[slot].record(main_stream)
       # get_next + train through common.function (the reference idiom: examples wrap
       # agent.train in common.function), i.e. the same captured step as `value`
-      out = fn()
+      out = fn()[0].loss
     loss_slots[slot:slot + 1].copy_(out.reshape(1), non_blocking=True)   # device -> pinned host
     loss_done[slot].record(main_stream)
     if read_prev:                                  # read the PREVIOUS step's loss while this one runs
