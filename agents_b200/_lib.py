@@ -98,8 +98,6 @@ SIGNATURES = {
     'b200rl_dqn_td_loss': [_P, _P, _P, _P, _P, _P, _P, _P, _P, c_i64, c_i64, c_i64, c_i64, c_i64,
                            c_f64, c_f64, c_int, c_f32, _P, _P, _P, _P, _P, _P],
     'b200rl_set_gemm_mode': [c_int],
-    'b200rl_tc_debug_buffer': [_P],
-    'b200rl_tc_debug_variant': [c_int],
     'b200rl_set_tc2_flags': [c_int],
     'b200rl_set_tile_scheduler': [c_int],
     'b200rl_tc2_trace_buffer': [_P],

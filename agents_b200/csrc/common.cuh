@@ -39,7 +39,7 @@ constexpr int kNumSMs = 148;  // B200: 2 dies x 74 SMs
 // stream be scheduled while this one runs.  With the wait first, ordering is exactly stream
 // order; what is gained is that the next grid's launch latency and block scheduling overlap this
 // grid's execution instead of following it (2-3 us per node in a captured step).
-// Kernels with a global-memory-free prologue (tc_gemm: barrier init, TMEM allocation) call
+// Kernels with a global-memory-free prologue (tc2_gemm: barrier init, TMEM allocation) call
 // pdl_launch_dependents() first and pdl_wait() after the prologue instead.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() {

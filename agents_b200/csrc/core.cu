@@ -34,7 +34,7 @@ int pdl_enabled() {
 extern "C" {
 
 const char* b200rl_last_error(void) { return b200rl::g_err; }
-int b200rl_version(void) { return 100; }
+int b200rl_version(void) { return 101; }
 int64_t b200rl_launch_count(void) { return b200rl::g_launches.load(); }
 
 int b200rl_set_pdl(int enabled) {

@@ -53,8 +53,8 @@ struct FastDiv {
 
 // Operand views.  Every view is separable: element (row, k) lives at row_off(row) + k_off(k),
 // where "row" is m for A views and n for B views.  kKContig says which index is contiguous in
-// memory (4 consecutive k can then be fetched with one 16-byte / 4-byte vector load when
-// vec4_ok()).  `at` is the scalar accessor used by the fp32 FFMA kernel.
+// memory.  `at` is the scalar accessor of the fp32 FFMA kernel; `addr` is the raw address the
+// tensor-core kernel copies 16-byte chunks from (tc2_gemm.cuh).
 struct ARow {
   const float* p;
   int64_t ld;
@@ -66,25 +66,19 @@ struct ARow {
   __device__ __forceinline__ int64_t row_off(int64_t m) const { return m * ld; }
   __device__ __forceinline__ int64_t k_off(int64_t k) const { return k; }
   __device__ __forceinline__ int64_t k_stride() const { return 1; }
-  __device__ __forceinline__ bool vec4_ok() const { return (ld & 3) == 0 && ((uintptr_t)p & 15) == 0; }
-  __device__ __forceinline__ float ld1(int64_t off) const { return p[off]; }
-  __device__ __forceinline__ float4 ld4(int64_t off) const { return *reinterpret_cast<const float4*>(p + off); }
   __device__ __forceinline__ const void* addr(int64_t off) const { return p + off; }
 };
 struct ACol {
   const float* p;
   int64_t ld;
   static constexpr bool kKContig = false;
-  static constexpr bool kTma2D = false;        // plain row-major [rows, K] matrix: TMA tile loads in tc2
+  static constexpr bool kTma2D = false;
   static constexpr bool kLinearK = true;      // k_off(k) == k * k_stride()
   static constexpr bool kExact = false;
   __device__ __forceinline__ float at(int64_t m, int64_t k) const { return p[k * ld + m]; }
   __device__ __forceinline__ int64_t row_off(int64_t m) const { return m; }
   __device__ __forceinline__ int64_t k_off(int64_t k) const { return k * ld; }
   __device__ __forceinline__ int64_t k_stride() const { return ld; }
-  __device__ __forceinline__ bool vec4_ok() const { return (ld & 3) == 0 && ((uintptr_t)p & 15) == 0; }
-  __device__ __forceinline__ float ld1(int64_t off) const { return p[off]; }
-  __device__ __forceinline__ float4 ld4(int64_t off) const { return *reinterpret_cast<const float4*>(p + off); }
   __device__ __forceinline__ const void* addr(int64_t off) const { return p + off; }
 };
 struct BRow {  // B(k, n) = p[k*ld + n]  (n contiguous)
@@ -92,16 +86,13 @@ struct BRow {  // B(k, n) = p[k*ld + n]  (n contiguous)
   int64_t ld;
   static constexpr bool kNContig = true;
   static constexpr bool kKContig = false;
-  static constexpr bool kTma2D = false;        // plain row-major [rows, K] matrix: TMA tile loads in tc2
+  static constexpr bool kTma2D = false;
   static constexpr bool kLinearK = true;      // k_off(k) == k * k_stride()
   static constexpr bool kExact = false;
   __device__ __forceinline__ float at(int64_t k, int64_t n) const { return p[k * ld + n]; }
   __device__ __forceinline__ int64_t row_off(int64_t n) const { return n; }
   __device__ __forceinline__ int64_t k_off(int64_t k) const { return k * ld; }
   __device__ __forceinline__ int64_t k_stride() const { return ld; }
-  __device__ __forceinline__ bool vec4_ok() const { return (ld & 3) == 0 && ((uintptr_t)p & 15) == 0; }
-  __device__ __forceinline__ float ld1(int64_t off) const { return p[off]; }
-  __device__ __forceinline__ float4 ld4(int64_t off) const { return *reinterpret_cast<const float4*>(p + off); }
   __device__ __forceinline__ const void* addr(int64_t off) const { return p + off; }
 };
 struct BCol {  // B(k, n) = p[n*ld + k]  (k contiguous)
@@ -116,9 +107,6 @@ struct BCol {  // B(k, n) = p[n*ld + k]  (k contiguous)
   __device__ __forceinline__ int64_t row_off(int64_t n) const { return n * ld; }
   __device__ __forceinline__ int64_t k_off(int64_t k) const { return k; }
   __device__ __forceinline__ int64_t k_stride() const { return 1; }
-  __device__ __forceinline__ bool vec4_ok() const { return (ld & 3) == 0 && ((uintptr_t)p & 15) == 0; }
-  __device__ __forceinline__ float ld1(int64_t off) const { return p[off]; }
-  __device__ __forceinline__ float4 ld4(int64_t off) const { return *reinterpret_cast<const float4*>(p + off); }
   __device__ __forceinline__ const void* addr(int64_t off) const { return p + off; }
 };
 
@@ -158,30 +146,10 @@ struct ConvView {
     return (int64_t)ky * g.in_row + r;
   }
   __device__ __forceinline__ float load(int64_t off) const { return cvt_in<T>(x[off], scale); }
-  __device__ __forceinline__ bool vec4_ok() const {
-    return (g.C & 3) == 0 && (g.in_img & 3) == 0 && ((uintptr_t)x & (4 * sizeof(T) - 1)) == 0;
-  }
-  __device__ __forceinline__ float4 load4(int64_t off) const;
-  // tensor-core path: x * (1/scale) instead of the IEEE division (differs by <= 1 ulp; the
-  // parity bar is 1e-5, and the division costs ~25 instructions per element in the producers)
-  __device__ __forceinline__ float load_fast(int64_t off) const;
 };
-template <>
-__device__ __forceinline__ float4 ConvView<float>::load4(int64_t off) const {
-  return *reinterpret_cast<const float4*>(x + off);
-}
-template <>
-__device__ __forceinline__ float4 ConvView<uint8_t>::load4(int64_t off) const {
-  const uchar4 u = *reinterpret_cast<const uchar4*>(x + off);
-  const float inv = __frcp_rn(scale);
-  return make_float4((float)u.x * inv, (float)u.y * inv, (float)u.z * inv, (float)u.w * inv);
-}
-template <>
-__device__ __forceinline__ float ConvView<float>::load_fast(int64_t off) const { return x[off]; }
-template <>
-__device__ __forceinline__ float ConvView<uint8_t>::load_fast(int64_t off) const {
-  return (float)x[off] * __frcp_rn(scale);
-}
+// fp32 im2col views of an fp32 or uint8 input (the latter with the reference's cast / scale).
+// `addr` hands the tensor-core kernel fp32 data, so it only compiles for T = float: uint8 inputs
+// reach that kernel through the raw views below.
 template <typename T>
 struct AConv {
   ConvView<T> v;
@@ -194,10 +162,7 @@ struct AConv {
   }
   __device__ __forceinline__ int64_t row_off(int64_t m) const { return v.pos_offset((uint32_t)m); }
   __device__ __forceinline__ int64_t k_off(int64_t k) const { return v.patch_offset((uint32_t)k); }
-  __device__ __forceinline__ bool vec4_ok() const { return v.vec4_ok(); }
-  __device__ __forceinline__ float ld1(int64_t off) const { return v.load_fast(off); }
-  __device__ __forceinline__ float4 ld4(int64_t off) const { return v.load4(off); }
-  __device__ __forceinline__ const void* addr(int64_t off) const { return v.x + off; }
+  __device__ __forceinline__ const float* addr(int64_t off) const { return v.x + off; }
 };
 template <typename T>
 struct AConvT {
@@ -211,29 +176,20 @@ struct AConvT {
   }
   __device__ __forceinline__ int64_t row_off(int64_t m) const { return v.patch_offset((uint32_t)m); }
   __device__ __forceinline__ int64_t k_off(int64_t k) const { return v.pos_offset((uint32_t)k); }
-  __device__ __forceinline__ bool vec4_ok() const { return v.vec4_ok(); }
-  __device__ __forceinline__ float ld1(int64_t off) const { return v.load_fast(off); }
-  __device__ __forceinline__ float4 ld4(int64_t off) const { return v.load4(off); }
-  __device__ __forceinline__ const void* addr(int64_t off) const { return v.x + off; }
+  __device__ __forceinline__ const float* addr(int64_t off) const { return v.x + off; }
 };
 
-// Raw uint8 pixel views for the tensor-core path: values 0..255 are exact in TF32, the 1/scale of
-// the reference's cast+/255 layer is applied to the accumulator in the epilogue instead.
+// Raw uint8 pixel views for the tensor-core kernel: values 0..255 are exact in TF32, the 1/scale of
+// the reference's cast+/255 layer is applied to the accumulator in the epilogue instead.  They
+// have no `at`, so they cannot be compiled into the FFMA kernel.
 struct AConvU8Raw {
   ConvView<uint8_t> v;
   static constexpr bool kKContig = true;
   static constexpr bool kTma2D = false;
   static constexpr bool kLinearK = false;
   static constexpr bool kExact = true;
-  __device__ __forceinline__ float at(int64_t m, int64_t k) const { return 0.f; }
   __device__ __forceinline__ int64_t row_off(int64_t m) const { return v.pos_offset((uint32_t)m); }
   __device__ __forceinline__ int64_t k_off(int64_t k) const { return v.patch_offset((uint32_t)k); }
-  __device__ __forceinline__ bool vec4_ok() const { return v.vec4_ok(); }
-  __device__ __forceinline__ float ld1(int64_t off) const { return (float)v.x[off]; }
-  __device__ __forceinline__ float4 ld4(int64_t off) const {
-    const uchar4 u = *reinterpret_cast<const uchar4*>(v.x + off);
-    return make_float4((float)u.x, (float)u.y, (float)u.z, (float)u.w);
-  }
   __device__ __forceinline__ const void* addr(int64_t off) const { return v.x + off; }
 };
 struct AConvTU8Raw {
@@ -242,15 +198,8 @@ struct AConvTU8Raw {
   static constexpr bool kTma2D = false;
   static constexpr bool kLinearK = false;
   static constexpr bool kExact = true;
-  __device__ __forceinline__ float at(int64_t m, int64_t k) const { return 0.f; }
   __device__ __forceinline__ int64_t row_off(int64_t m) const { return v.patch_offset((uint32_t)m); }
   __device__ __forceinline__ int64_t k_off(int64_t k) const { return v.pos_offset((uint32_t)k); }
-  __device__ __forceinline__ bool vec4_ok() const { return v.vec4_ok(); }
-  __device__ __forceinline__ float ld1(int64_t off) const { return (float)v.x[off]; }
-  __device__ __forceinline__ float4 ld4(int64_t off) const {
-    const uchar4 u = *reinterpret_cast<const uchar4*>(v.x + off);
-    return make_float4((float)u.x, (float)u.y, (float)u.z, (float)u.w);
-  }
   __device__ __forceinline__ const void* addr(int64_t off) const { return v.x + off; }
 };
 
@@ -275,7 +224,6 @@ __device__ __forceinline__ float dact(float y, float g, int act) {
 }
 
 }  // namespace b200rl
-#include "tc_gemm.cuh"
 #include "tc2_gemm.cuh"
 namespace b200rl {
 
@@ -905,67 +853,17 @@ static int gemm_mode() {
   return g_gemm_mode;
 }
 
-template <int BN, int STAGES, int PASSES, int EPI, class AL, class BL>
-static int launch_tc_cfg(const AL& a, const BL& b, const GemmArgs& g, const tc::EpiArgs& epi) {
-  using L = tc::SmemLayout<BN, STAGES, PASSES, AL::kExact>;
-  auto kernel = tc::tc_gemm_kernel<BN, STAGES, PASSES, EPI, AL, BL>;
-  static bool configured = false;
-  if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         L::kBytes);
-    if (e != cudaSuccess) {
-      set_error("tc_gemm: cannot set dynamic smem to %d: %s", L::kBytes, cudaGetErrorString(e));
-      return B200RL_ERR_CUDA;
-    }
-    configured = true;
+// ---- tensor-core (tc2) kernel: eligibility and launch ------------------------------------------
+// B200RL_TC2_FLAGS: A/B switches of tc2_gemm.cuh (as b200rl_set_tc2_flags), read at the first launch.
+static void tc2_env_flags() {
+  static bool done = false;
+  if (done) return;
+  done = true;
+  const char* f = getenv("B200RL_TC2_FLAGS");
+  if (f) {
+    const int flags = atoi(f);
+    cudaMemcpyToSymbol(tc2::g_tc2_flags, &flags, sizeof(flags));
   }
-  const int64_t tm = (g.M + tc::kBM - 1) / tc::kBM, tn = (g.N + BN - 1) / BN;
-  const int64_t tiles = tm * tn;
-  int splits = 1;
-  const int64_t target = (BN <= 64 ? 2 : 1) * (int64_t)kNumSMs;  // resident CTAs on the chip
-  if (tiles < target && g.K >= 8 * tc::kBK && (g.ws != nullptr || EPI != tc::EPI_STORE)) {
-    int64_t want = target / tiles;  // only split when a whole extra set of CTAs fits on the chip
-    int64_t max_by_k = g.K / (4 * tc::kBK);
-    int64_t max_by_ws = EPI != tc::EPI_STORE ? 65535 : g.ws_bytes / (int64_t)(g.M * g.N * sizeof(float));
-    int64_t s = want < max_by_k ? want : max_by_k;
-    if (s > max_by_ws) s = max_by_ws;
-    if (s > 65535) s = 65535;
-    if (s >= 2) splits = (int)s;
-  }
-  int64_t kps = (g.K + splits - 1) / splits;
-  kps = (kps + tc::kBK - 1) / tc::kBK * tc::kBK;
-  splits = (int)((g.K + kps - 1) / kps);
-  if (splits < 1) splits = 1;
-  B200RL_CHECK_ARG(tm <= 65535, "tc_gemm: M too large for grid.y (%lld tiles)", (long long)tm);
-  dim3 grid((unsigned)tn, (unsigned)tm, (unsigned)splits);
-  B200RL_LAUNCH(kernel, grid, tc::kThreads, L::kBytes, g.st, a, b, epi, g.C, g.bias, g.M, g.N, g.K, g.act, g.beta, splits, kps, (float*)g.ws, g.out_scale);
-  B200RL_CHECK_LAUNCH("tc_gemm");
-  if (splits > 1 && EPI == tc::EPI_STORE) {
-    const int64_t MN = g.M * g.N;
-    B200RL_LAUNCH(splitk_reduce_kernel, (unsigned)((MN + 255) / 256), 256, 0, g.st, (const float*)g.ws, g.C, g.bias, MN, g.N, splits, g.act, g.beta, g.mask);
-    B200RL_CHECK_LAUNCH("splitk_reduce");
-  }
-  return B200RL_OK;
-}
-
-
-// ---- second-generation (persistent, cp.async) kernel: eligibility and launch ---------------------
-// tc2 only takes operands whose every 16-byte chunk is contiguous and aligned in global memory;
-// everything else stays on tc_gemm_kernel (which has the scalar paths).
-static int g_tc2_host_flags = 0;   // bit 1: route everything to the first-generation kernel
-static int tc2_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("B200RL_TC2");
-    v = e ? atoi(e) : 1;
-    const char* f = getenv("B200RL_TC2_FLAGS");    // profiles/: A/B switches of tc2_gemm.cuh
-    if (f) {
-      const int flags = atoi(f);
-      g_tc2_host_flags = flags;
-      cudaMemcpyToSymbol(tc2::g_tc2_flags, &flags, sizeof(flags));
-    }
-  }
-  return v && !(g_tc2_host_flags & 2);
 }
 // Work distribution of the persistent GEMM: 0 = static striding (a few per cent faster when the
 // kernel has the GPU to itself), 1 = dynamic (global counter): CTAs whose SM is busy with a
@@ -980,6 +878,8 @@ static bool tile_scheduler_dynamic() {
   }
   return g_tile_sched != 0;
 }
+// tc2 only takes operands whose every 16-byte chunk is contiguous and aligned in global memory.
+// There is no overload for the fp32-cast uint8 conv views: they never take the tensor route.
 static bool al16(const void* p) { return ((uintptr_t)p & 15) == 0; }
 static bool tc2_ok(const ARow& v, int64_t rows, int64_t K) { return (v.ld & 3) == 0 && al16(v.p) && (K & 3) == 0; }
 static bool tc2_ok(const BCol& v, int64_t rows, int64_t K) { return (v.ld & 3) == 0 && al16(v.p) && (K & 3) == 0; }
@@ -997,8 +897,6 @@ static bool conv_u8_ok(const ConvView<uint8_t>& v) {
 }
 static bool tc2_ok(const AConvU8Raw& v, int64_t rows, int64_t K) { return conv_u8_ok(v.v) && (K & 15) == 0; }
 static bool tc2_ok(const AConvTU8Raw& v, int64_t rows, int64_t K) { return conv_u8_ok(v.v) && (rows & 15) == 0; }
-template <class V>
-static bool tc2_ok(const V&, int64_t, int64_t) { return false; }   // AConv<uint8_t> with the exact division etc.
 
 
 // ---- TMA tensor maps for plain 2-D operands (tc2) ---------------------------------------------
@@ -1074,8 +972,8 @@ static const void* view_base(const ARow& v) { return v.p; }
 static const void* view_base(const ACol& v) { return v.p; }
 static const void* view_base(const BRow& v) { return v.p; }
 static const void* view_base(const BCol& v) { return v.p; }
-template <class T> static const void* view_base(const AConv<T>& v) { return v.v.x; }
-template <class T> static const void* view_base(const AConvT<T>& v) { return v.v.x; }
+static const void* view_base(const AConv<float>& v) { return v.v.x; }
+static const void* view_base(const AConvT<float>& v) { return v.v.x; }
 static const void* view_base(const AConvU8Raw& v) { return v.v.x; }
 static const void* view_base(const AConvTU8Raw& v) { return v.v.x; }
 
@@ -1089,8 +987,8 @@ struct Tc2Pair {
 };
 
 template <int BN, int PASSES, int EPI, class AL, class BL>
-static int launch_tc2_cfg(const AL& a, const BL& b, const GemmArgs& g, const tc::EpiArgs& epi,
-                          const Tc2Pair<AL, BL>* pair = nullptr) {
+static int launch_tc2_cfg(const AL& a, const BL& b, const GemmArgs& g, const tc2::EpiArgs& epi,
+                          const Tc2Pair<AL, BL>* pair) {
   using L = tc2::Layout<BN, PASSES, AL::kExact>;
   auto kernel = tc2::tc2_gemm_kernel<BN, PASSES, EPI, AL, BL>;
   static bool configured = false;
@@ -1103,28 +1001,29 @@ static int launch_tc2_cfg(const AL& a, const BL& b, const GemmArgs& g, const tc:
     }
     configured = true;
   }
-  const int64_t tm1 = (g.M + tc::kBM - 1) / tc::kBM, tn = (g.N + BN - 1) / BN;
+  tc2_env_flags();
+  const int64_t tm1 = (g.M + tc2::kBM - 1) / tc2::kBM, tn = (g.N + BN - 1) / BN;
   const int64_t tm = pair ? 2 * tm1 : tm1;
   const int64_t tiles = tm * tn;
   int splits = 1;
   const int64_t target = kNumSMs;                  // one persistent CTA per SM
-  if (tiles < target && g.K >= 8 * tc::kBK && (g.ws != nullptr || EPI != tc::EPI_STORE)) {
+  if (tiles < target && g.K >= 8 * tc2::kBK && (g.ws != nullptr || EPI != tc2::EPI_STORE)) {
     int64_t want = target / tiles;
-    int64_t max_by_k = g.K / (4 * tc::kBK);
-    int64_t max_by_ws = EPI != tc::EPI_STORE ? 65535 : g.ws_bytes / (int64_t)((pair ? 2 : 1) * g.M * g.N * sizeof(float));
+    int64_t max_by_k = g.K / (4 * tc2::kBK);
+    int64_t max_by_ws = EPI != tc2::EPI_STORE ? 65535 : g.ws_bytes / (int64_t)((pair ? 2 : 1) * g.M * g.N * sizeof(float));
     int64_t s = want < max_by_k ? want : max_by_k;
     if (s > max_by_ws) s = max_by_ws;
     if (s >= 2) splits = (int)s;
   }
   int64_t kps = (g.K + splits - 1) / splits;
-  kps = (kps + tc::kBK - 1) / tc::kBK * tc::kBK;
+  kps = (kps + tc2::kBK - 1) / tc2::kBK * tc2::kBK;
   splits = (int)((g.K + kps - 1) / kps);
   if (splits < 1) splits = 1;
   const int64_t total = tiles * splits;
   B200RL_CHECK_ARG(total < (1ll << 31), "tc2_gemm: too many work items");
   const unsigned grid = (unsigned)(total < kNumSMs ? total : kNumSMs);
   CUtensorMap tmA, tmB, tmA2, tmB2;
-  int rc = tmap_for(a, g.M, g.K, tc::kBM, &tmA);
+  int rc = tmap_for(a, g.M, g.K, tc2::kBM, &tmA);
   if (rc) return rc;
   rc = tmap_for(b, g.N, g.K, BN, &tmB);
   if (rc) return rc;
@@ -1132,7 +1031,7 @@ static int launch_tc2_cfg(const AL& a, const BL& b, const GemmArgs& g, const tc:
   tmB2 = tmB;
   tc2::PairArgs pa{tm1, 0, 0, 0, 0};
   if (pair) {
-    rc = tmap_for(pair->a, g.M, g.K, tc::kBM, &tmA2);
+    rc = tmap_for(pair->a, g.M, g.K, tc2::kBM, &tmA2);
     if (rc) return rc;
     rc = tmap_for(pair->b, g.N, g.K, BN, &tmB2);
     if (rc) return rc;
@@ -1144,14 +1043,14 @@ static int launch_tc2_cfg(const AL& a, const BL& b, const GemmArgs& g, const tc:
   // epilogue-bound shapes (col2im scatter-add, short K loops) get all eight epilogue warps
   static const int epi_env = [] { const char* e = getenv("B200RL_TC2_EPI_WARPS"); return e ? atoi(e) : 0; }();
   const int epi_warps = (epi_env == 4 || epi_env == 8) ? epi_env
-                        : (EPI == tc::EPI_COL2IM || EPI == tc::EPI_COL2IM_MERGE || kps <= 224) ? 8 : 4;
+                        : (EPI == tc2::EPI_COL2IM || EPI == tc2::EPI_COL2IM_MERGE || kps <= 224) ? 8 : 4;
   // dynamic work distribution (b200rl_set_tile_scheduler) when a CTA has more than one item
   static int sched_seq = 0;
   int sched_slot = -1;
   if (total > grid && tile_scheduler_dynamic()) sched_slot = (sched_seq++) & (tc2::kSchedSlots - 1);
   B200RL_LAUNCH(kernel, grid, tc2::kThreads, L::kBytes, g.st, a, b, epi, g.C, g.bias, g.M, g.N, g.K, g.act, g.beta, splits, kps, (float*)g.ws, g.out_scale, tm, tn, epi_warps, sched_slot, pa, tmA, tmB, tmA2, tmB2);
   B200RL_CHECK_LAUNCH("tc2_gemm");
-  if (splits > 1 && EPI == tc::EPI_STORE) {
+  if (splits > 1 && EPI == tc2::EPI_STORE) {
     const int64_t MN = g.M * g.N;
     B200RL_LAUNCH(splitk_reduce_kernel, (unsigned)((MN + 255) / 256), 256, 0, g.st, (const float*)g.ws, g.C, g.bias, MN, g.N, splits, g.act, g.beta, g.mask);
     B200RL_CHECK_LAUNCH("splitk_reduce");
@@ -1163,55 +1062,35 @@ static int launch_tc2_cfg(const AL& a, const BL& b, const GemmArgs& g, const tc:
   return B200RL_OK;
 }
 
-// BN by N like the first-generation dispatch
-template <int PASSES, int EPI, class AL, class BL>
-static int launch_tc2(const AL& a, const BL& b, const GemmArgs& g, const tc::EpiArgs& epi,
-                      const Tc2Pair<AL, BL>* pair = nullptr) {
-  if (g.N <= 32) return launch_tc2_cfg<32, PASSES, EPI>(a, b, g, epi, pair);
-  if (g.N <= 64) return launch_tc2_cfg<64, PASSES, EPI>(a, b, g, epi, pair);
-  return launch_tc2_cfg<128, PASSES, EPI>(a, b, g, epi, pair);
-}
-template <class V> struct Tc2Capable { static constexpr bool value = true; };
-template <> struct Tc2Capable<AConv<uint8_t>> { static constexpr bool value = false; };
-template <> struct Tc2Capable<AConvT<uint8_t>> { static constexpr bool value = false; };
+// ---- one route rule for every dense / conv GEMM ------------------------------------------------
+// Tensor route (tc2_gemm_kernel) when the GEMM mode allows it, the problem fills a tensor-core tile
+// well enough, and both operand views can be moved as aligned 16-byte chunks; every other shape
+// takes the fp32 FFMA kernel (launch_ffma).
 template <class AL, class BL>
-static bool use_tc2(const AL& a, const BL& b, const GemmArgs& g) {
-  return tc2_enabled() && tc2_ok(a, g.M, g.K) && tc2_ok(b, g.N, g.K);
+static bool tensor_route(const AL& a, const BL& b, const GemmArgs& g) {
+  return gemm_mode() != 0 && g.N >= 16 && g.M >= 32 && g.K >= 8 && tc2_ok(a, g.M, g.K) &&
+         tc2_ok(b, g.N, g.K);
 }
 
-template <int PASSES, class AL, class BL>
-static int launch_tc(const AL& a, const BL& b, const GemmArgs& g) {
-  tc::EpiArgs none{};
-  none.mask = g.mask;
-  B200RL_CHECK_ARG(!(g.mask.y && g.beta), "gemm: an input-gradient mask cannot be combined with accumulation");
-  if constexpr (Tc2Capable<AL>::value) {
-    if (use_tc2(a, b, g)) return launch_tc2<PASSES, tc::EPI_STORE>(a, b, g, none);
+// 3xTF32 in mode 1, 1xTF32 in mode 2.  BN by N; the col2im epilogues always use 128-column tiles
+// (the merged one pairs columns 64 apart inside a tile).
+template <int EPI, class AL, class BL>
+static int launch_tensor(const AL& a, const BL& b, const GemmArgs& g, const tc2::EpiArgs& epi,
+                         const Tc2Pair<AL, BL>* pair = nullptr) {
+  constexpr bool kCol2im = EPI == tc2::EPI_COL2IM || EPI == tc2::EPI_COL2IM_MERGE;
+  const bool one_pass = gemm_mode() == 2;
+  if constexpr (!kCol2im) {
+    if (g.N <= 32) return one_pass ? launch_tc2_cfg<32, 1, EPI>(a, b, g, epi, pair)
+                                   : launch_tc2_cfg<32, 3, EPI>(a, b, g, epi, pair);
+    if (g.N <= 64) return one_pass ? launch_tc2_cfg<64, 1, EPI>(a, b, g, epi, pair)
+                                   : launch_tc2_cfg<64, 3, EPI>(a, b, g, epi, pair);
   }
-  if (g.N <= 32) return launch_tc_cfg<32, (AL::kExact ? 4 : 2), PASSES, tc::EPI_STORE>(a, b, g, none);  // <= 96 KB -> 2 CTAs/SM
-  if (g.N <= 64) return launch_tc_cfg<64, 2, PASSES, tc::EPI_STORE>(a, b, g, none);  // 96 KB -> 2 CTAs/SM
-  return launch_tc_cfg<128, 3, PASSES, tc::EPI_STORE>(a, b, g, none);
+  return one_pass ? launch_tc2_cfg<128, 1, EPI>(a, b, g, epi, pair)
+                  : launch_tc2_cfg<128, 3, EPI>(a, b, g, epi, pair);
 }
 
-// Weight-gradient GEMMs (no bias / activation): in tensor-core mode the split-K partials are
-// accumulated with red.global.add straight into the (zeroed) gradient instead of going through
-// a workspace + reduce kernel.  Summation order across splits is not fixed.
-// `db` (optional): bias gradient = column sums of B; when the tensor-core path takes the GEMM and
-// B is an MN-major view the sums are accumulated by the producers of the same kernel and
-// *db_fused is set, otherwise the caller runs the separate column-sum kernels.
 template <class AL, class BL>
-static int launch_grad_gemm(const AL& a, const BL& b, const GemmArgs& g, float* db = nullptr,
-                            bool* db_fused = nullptr);
-
-template <class AL, class BL>
-static int launch_gemm(const AL& a, const BL& b, const GemmArgs& g) {
-  if (g.M <= 0 || g.N <= 0) return B200RL_OK;
-  B200RL_CHECK_ARG(g.K > 0, "gemm: K must be > 0");
-  B200RL_CHECK_ARG(g.M < (1ll << 31) && g.N < (1ll << 31) && g.K < (1ll << 31), "gemm: dims");
-  const int mode = gemm_mode();
-  if (mode != 0 && g.N >= 16 && g.M >= 32 && g.K >= 8) {
-    if (mode == 2) return launch_tc<1>(a, b, g);
-    return launch_tc<3>(a, b, g);
-  }
+static int launch_ffma(const AL& a, const BL& b, const GemmArgs& g) {
   if (g.N <= 32) return launch_gemm_cfg<128, 32, 4, 4>(a, b, g);
   if (g.N <= 64) {
     if (g.M >= 4096) return launch_gemm_cfg<128, 64, 8, 4>(a, b, g);
@@ -1222,12 +1101,26 @@ static int launch_gemm(const AL& a, const BL& b, const GemmArgs& g) {
   return launch_gemm_cfg<64, 64, 4, 4>(a, b, g);
 }
 
+// C = act(A @ B + bias) (* act'(mask)) (+ C when beta)
 template <class AL, class BL>
-static int launch_grad_gemm(const AL& a, const BL& b, const GemmArgs& g, float* db, bool* db_fused) {
-  const int mode = gemm_mode();
-  if (db_fused) *db_fused = false;
-  if (mode == 0 || g.N < 16 || g.M < 32 || g.K < 8 || g.bias != nullptr || g.act != B200RL_ACT_NONE)
-    return launch_gemm(a, b, g);
+static int launch_gemm(const AL& a, const BL& b, const GemmArgs& g) {
+  if (g.M <= 0 || g.N <= 0) return B200RL_OK;
+  B200RL_CHECK_ARG(g.K > 0, "gemm: K must be > 0");
+  B200RL_CHECK_ARG(g.M < (1ll << 31) && g.N < (1ll << 31) && g.K < (1ll << 31), "gemm: dims");
+  if (!tensor_route(a, b, g)) return launch_ffma(a, b, g);
+  B200RL_CHECK_ARG(!(g.mask.y && g.beta), "gemm: an input-gradient mask cannot be combined with accumulation");
+  tc2::EpiArgs epi{};
+  epi.mask = g.mask;
+  return launch_tensor<tc2::EPI_STORE>(a, b, g, epi);
+}
+
+// Weight-gradient GEMM (no bias / activation) on the tensor route: the split-K partials are
+// accumulated with red.global.add straight into the (zeroed) gradient instead of going through a
+// workspace + reduce kernel; summation order across splits is not fixed.  `db` (optional): bias
+// gradient = column sums of B; for an MN-major B view they are accumulated by the converters of
+// the same kernel and *db_fused is set, otherwise the caller runs the separate column-sum kernels.
+template <class AL, class BL>
+static int launch_grad_tensor(const AL& a, const BL& b, const GemmArgs& g, float* db, bool* db_fused) {
   const bool fuse_db = db != nullptr && !BL::kKContig && fuse_bias_grad();
   if (!g.beta) {
     cudaError_t e = cudaMemsetAsync(g.C, 0, (size_t)(g.M * g.N) * sizeof(float), g.st);
@@ -1237,27 +1130,17 @@ static int launch_grad_gemm(const AL& a, const BL& b, const GemmArgs& g, float* 
       return B200RL_ERR_CUDA;
     }
   }
-  tc::EpiArgs none{};
-  if (fuse_db) {
-    none.colsum = db;
-    if (db_fused) *db_fused = true;
-  }
-  if constexpr (Tc2Capable<AL>::value) {
-    if (use_tc2(a, b, g)) {
-      if (mode == 2) return launch_tc2<1, tc::EPI_ATOMIC>(a, b, g, none);
-      return launch_tc2<3, tc::EPI_ATOMIC>(a, b, g, none);
-    }
-  }
-  if (mode == 2) {
-    if (g.N <= 32) return launch_tc_cfg<32, (AL::kExact ? 4 : 2), 1, tc::EPI_ATOMIC>(a, b, g, none);
-    if (g.N <= 64) return launch_tc_cfg<64, 2, 1, tc::EPI_ATOMIC>(a, b, g, none);
-    return launch_tc_cfg<128, 3, 1, tc::EPI_ATOMIC>(a, b, g, none);
-  }
-  if (g.N <= 32) return launch_tc_cfg<32, (AL::kExact ? 4 : 2), 3, tc::EPI_ATOMIC>(a, b, g, none);
-  if (g.N <= 64) return launch_tc_cfg<64, 2, 3, tc::EPI_ATOMIC>(a, b, g, none);
-  return launch_tc_cfg<128, 3, 3, tc::EPI_ATOMIC>(a, b, g, none);
+  tc2::EpiArgs epi{};
+  if (fuse_db) epi.colsum = db;
+  *db_fused = fuse_db;
+  return launch_tensor<tc2::EPI_ATOMIC>(a, b, g, epi);
 }
-
+template <class AL, class BL>
+static int launch_grad_gemm(const AL& a, const BL& b, const GemmArgs& g, float* db, bool* db_fused) {
+  *db_fused = false;
+  if (!tensor_route(a, b, g)) return launch_gemm(a, b, g);   // FFMA route
+  return launch_grad_tensor(a, b, g, db, db_fused);
+}
 
 // ---- skinny-head dispatch (N <= 16) ----------------------------------------------------------
 static bool skinny_ok(int64_t M, int64_t K, int64_t N) {
@@ -1345,50 +1228,27 @@ static int make_geom(const b200rl_conv_t* c, ConvGeom& g) {
 using namespace b200rl;
 
 // Forward pass of TWO layers of identical shape in one launch (DQN: the online network on
-// obs[:, 0] and the target network on obs[:, T-1]).  Falls back to two launches whenever the
-// persistent tensor-core kernel does not take the shape.
+// obs[:, 0] and the target network on obs[:, T-1]): when both problems take the tensor route and
+// both or neither have a bias.  Otherwise the callers make two single calls.
 static int pair_fwd_enabled() {
   static const int v = [] { const char* e = getenv("B200RL_PAIR_FWD"); return e ? atoi(e) : 1; }();
   return v;
 }
 template <class AL, class BL>
-static int launch_fwd_pair(const AL& a1, const BL& b1, const GemmArgs& g1, const AL& a2,
-                           const BL& b2, const GemmArgs& g2) {
-  const int mode = gemm_mode();
-  if constexpr (Tc2Capable<AL>::value) {
-    if (pair_fwd_enabled() && mode != 0 && g1.N >= 16 && g1.M >= 32 && g1.K >= 8 &&
-        use_tc2(a1, b1, g1) && use_tc2(a2, b2, g2) && (g1.bias == nullptr) == (g2.bias == nullptr)) {
-      tc::EpiArgs none{};
-      Tc2Pair<AL, BL> p{a2, b2, g2.C, g2.bias};
-      if (mode == 2) return launch_tc2<1, tc::EPI_STORE>(a1, b1, g1, none, &p);
-      return launch_tc2<3, tc::EPI_STORE>(a1, b1, g1, none, &p);
-    }
-  }
-  int rc = launch_gemm(a1, b1, g1);
-  if (rc) return rc;
-  return launch_gemm(a2, b2, g2);
+static bool pair_route(const AL& a1, const BL& b1, const GemmArgs& g1, const AL& a2, const BL& b2,
+                       const GemmArgs& g2) {
+  return pair_fwd_enabled() && tensor_route(a1, b1, g1) && tensor_route(a2, b2, g2) &&
+         (g1.bias == nullptr) == (g2.bias == nullptr);
+}
+template <class AL, class BL>
+static int launch_pair(const AL& a1, const BL& b1, const GemmArgs& g1, const AL& a2, const BL& b2,
+                       const GemmArgs& g2) {
+  const Tc2Pair<AL, BL> p{a2, b2, g2.C, g2.bias};
+  return launch_tensor<tc2::EPI_STORE>(a1, b1, g1, tc2::EpiArgs{}, &p);
 }
 
 
 extern "C" {
-
-int b200rl_tc_debug_buffer(long long* dev_buf) {
-  cudaError_t e = cudaMemcpyToSymbol(tc::g_tc_dbg, &dev_buf, sizeof(dev_buf));
-  if (e != cudaSuccess) {
-    set_error("tc_debug_buffer: %s", cudaGetErrorString(e));
-    return B200RL_ERR_CUDA;
-  }
-  return B200RL_OK;
-}
-
-int b200rl_tc_debug_variant(int v) {
-  cudaError_t e = cudaMemcpyToSymbol(tc::g_tc_variant, &v, sizeof(v));
-  if (e != cudaSuccess) {
-    set_error("tc_debug_variant: %s", cudaGetErrorString(e));
-    return B200RL_ERR_CUDA;
-  }
-  return B200RL_OK;
-}
 
 int b200rl_tc2_trace_buffer(long long* dev_buf) {
   cudaError_t e = cudaMemcpyToSymbol(tc2::g_tc2_trace, &dev_buf, sizeof(dev_buf));
@@ -1405,7 +1265,6 @@ int b200rl_set_tile_scheduler(int dynamic) {
 }
 
 int b200rl_set_tc2_flags(int flags) {
-  g_tc2_host_flags = flags;
   cudaError_t e = cudaMemcpyToSymbol(tc2::g_tc2_flags, &flags, sizeof(flags));
   if (e != cudaSuccess) {
     set_error("set_tc2_flags: %s", cudaGetErrorString(e));
@@ -1483,9 +1342,14 @@ int b200rl_dense_fwd_pair(const float* X1, const float* X2, int64_t ldx, const f
     if (rc) return rc;
     return b200rl_dense_fwd(X2, ldx, W2, bias2, Y2, M, K, N, act, workspace, ws_bytes, stream);
   }
-  GemmArgs g1{Y1, bias1, M, N, K, act, 0, workspace, ws_bytes, (cudaStream_t)stream};
-  GemmArgs g2{Y2, bias2, M, N, K, act, 0, workspace, ws_bytes, (cudaStream_t)stream};
-  return launch_fwd_pair(ARow{X1, ldx ? ldx : K}, BRow{W1, N}, g1, ARow{X2, ldx ? ldx : K}, BRow{W2, N}, g2);
+  const GemmArgs g1{Y1, bias1, M, N, K, act, 0, workspace, ws_bytes, (cudaStream_t)stream};
+  const GemmArgs g2{Y2, bias2, M, N, K, act, 0, workspace, ws_bytes, (cudaStream_t)stream};
+  const ARow a1{X1, ldx ? ldx : K}, a2{X2, ldx ? ldx : K};
+  const BRow b1{W1, N}, b2{W2, N};
+  if (pair_route(a1, b1, g1, a2, b2, g2)) return launch_pair(a1, b1, g1, a2, b2, g2);
+  int rc = launch_gemm(a1, b1, g1);
+  if (rc) return rc;
+  return launch_gemm(a2, b2, g2);
 }
 
 int b200rl_dense_bwd(const float* X, int64_t ldx, const float* W, const float* dY, float* dX,
@@ -1556,17 +1420,16 @@ int b200rl_conv2d_fwd(const void* X, int x_is_u8, float x_scale, const float* Wt
   if (rc) return rc;
   const int64_t M = (int64_t)c->N * cg.OH * cg.OW, K = (int64_t)c->KH * c->KW * c->C;
   GemmArgs g{Y, bias, M, c->F, K, act, 0, workspace, ws_bytes, (cudaStream_t)stream};
+  const BRow w{Wt, c->F};
   if (x_is_u8) {
-    if (gemm_mode() == 1 && c->F >= 16 && M >= 32 && K >= 8) {   // raw pixels, 2-pass 3xTF32
-      g.out_scale = 1.f / x_scale;
-      AConvU8Raw a{ConvView<uint8_t>{(const uint8_t*)X, cg, x_scale}};
-      return launch_tc<3>(a, BRow{Wt, c->F}, g);
-    }
-    AConv<uint8_t> a{ConvView<uint8_t>{(const uint8_t*)X, cg, x_scale}};
-    return launch_gemm(a, BRow{Wt, c->F}, g);
+    // raw pixels on the tensor route (1/x_scale applied to the accumulator), the reference's exact
+    // cast and division on the FFMA route
+    const ConvView<uint8_t> v{(const uint8_t*)X, cg, x_scale};
+    if (!tensor_route(AConvU8Raw{v}, w, g)) return launch_ffma(AConv<uint8_t>{v}, w, g);
+    g.out_scale = 1.f / x_scale;
+    return launch_tensor<tc2::EPI_STORE>(AConvU8Raw{v}, w, g, tc2::EpiArgs{});
   }
-  AConv<float> a{ConvView<float>{(const float*)X, cg, 1.f}};
-  return launch_gemm(a, BRow{Wt, c->F}, g);
+  return launch_gemm(AConv<float>{ConvView<float>{(const float*)X, cg, 1.f}}, w, g);
 }
 
 int b200rl_conv2d_fwd_pair(const void* X1, const void* X2, int x_is_u8, float x_scale,
@@ -1579,30 +1442,23 @@ int b200rl_conv2d_fwd_pair(const void* X1, const void* X2, int x_is_u8, float x_
   if (rc) return rc;
   const int64_t M = (int64_t)c->N * cg.OH * cg.OW, K = (int64_t)c->KH * c->KW * c->C;
   GemmArgs g1{Y1, bias1, M, c->F, K, act, 0, workspace, ws_bytes, (cudaStream_t)stream};
-  GemmArgs g2{Y2, bias2, M, c->F, K, act, 0, workspace, ws_bytes, (cudaStream_t)stream};
+  const GemmArgs g2{Y2, bias2, M, c->F, K, act, 0, workspace, ws_bytes, (cudaStream_t)stream};
+  const BRow b1{Wt1, c->F}, b2{Wt2, c->F};
   if (x_is_u8) {
-    if (gemm_mode() == 1 && c->F >= 16 && M >= 32 && K >= 8) {   // raw pixels, 2-pass 3xTF32
-      g1.out_scale = g2.out_scale = 1.f / x_scale;
-      AConvU8Raw a1{ConvView<uint8_t>{(const uint8_t*)X1, cg, x_scale}};
-      AConvU8Raw a2{ConvView<uint8_t>{(const uint8_t*)X2, cg, x_scale}};
-      const BRow b1{Wt1, c->F}, b2{Wt2, c->F};
-      if (pair_fwd_enabled() && use_tc2(a1, b1, g1) && use_tc2(a2, b2, g2) &&
-          (bias1 == nullptr) == (bias2 == nullptr)) {
-        tc::EpiArgs none{};
-        Tc2Pair<AConvU8Raw, BRow> p{a2, b2, Y2, bias2};
-        return launch_tc2<3, tc::EPI_STORE>(a1, b1, g1, none, &p);
-      }
-      rc = launch_tc<3>(a1, b1, g1);
-      if (rc) return rc;
-      return launch_tc<3>(a2, b2, g2);
+    const AConvU8Raw a1{ConvView<uint8_t>{(const uint8_t*)X1, cg, x_scale}};
+    const AConvU8Raw a2{ConvView<uint8_t>{(const uint8_t*)X2, cg, x_scale}};
+    if (pair_route(a1, b1, g1, a2, b2, g2)) {
+      g1.out_scale = 1.f / x_scale;
+      return launch_pair(a1, b1, g1, a2, b2, g2);
     }
-    rc = b200rl_conv2d_fwd(X1, x_is_u8, x_scale, Wt1, bias1, Y1, c, act, workspace, ws_bytes, stream);
-    if (rc) return rc;
-    return b200rl_conv2d_fwd(X2, x_is_u8, x_scale, Wt2, bias2, Y2, c, act, workspace, ws_bytes, stream);
+  } else {
+    const AConv<float> a1{ConvView<float>{(const float*)X1, cg, 1.f}};
+    const AConv<float> a2{ConvView<float>{(const float*)X2, cg, 1.f}};
+    if (pair_route(a1, b1, g1, a2, b2, g2)) return launch_pair(a1, b1, g1, a2, b2, g2);
   }
-  AConv<float> a1{ConvView<float>{(const float*)X1, cg, 1.f}};
-  AConv<float> a2{ConvView<float>{(const float*)X2, cg, 1.f}};
-  return launch_fwd_pair(a1, BRow{Wt1, c->F}, g1, a2, BRow{Wt2, c->F}, g2);
+  rc = b200rl_conv2d_fwd(X1, x_is_u8, x_scale, Wt1, bias1, Y1, c, act, workspace, ws_bytes, stream);
+  if (rc) return rc;
+  return b200rl_conv2d_fwd(X2, x_is_u8, x_scale, Wt2, bias2, Y2, c, act, workspace, ws_bytes, stream);
 }
 
 int b200rl_conv2d_bwd(const void* X, int x_is_u8, float x_scale, const float* Wt,
@@ -1623,16 +1479,17 @@ int b200rl_conv2d_bwd(const void* X, int x_is_u8, float x_scale, const float* Wt
   bool db_fused = false;
   if (dW) {  // dW[K,F] = im2col(X)^T @ dY
     GemmArgs g{dW, nullptr, K, F, M, B200RL_ACT_NONE, accumulate, workspace, ws_bytes, st};
-    if (x_is_u8 && gemm_mode() == 1 && F >= 16 && K >= 32 && M >= 8) {
-      g.out_scale = 1.f / x_scale;
-      AConvTU8Raw a{ConvView<uint8_t>{(const uint8_t*)X, cg, x_scale}};
-      rc = launch_grad_gemm(a, BRow{dY, F}, g, db, &db_fused);
-    } else if (x_is_u8) {
-      AConvT<uint8_t> a{ConvView<uint8_t>{(const uint8_t*)X, cg, x_scale}};
-      rc = launch_gemm(a, BRow{dY, F}, g);
+    const BRow dy{dY, F};
+    if (x_is_u8) {   // the two views of b200rl_conv2d_fwd
+      const ConvView<uint8_t> v{(const uint8_t*)X, cg, x_scale};
+      if (tensor_route(AConvTU8Raw{v}, dy, g)) {
+        g.out_scale = 1.f / x_scale;
+        rc = launch_grad_tensor(AConvTU8Raw{v}, dy, g, db, &db_fused);
+      } else {
+        rc = launch_ffma(AConvT<uint8_t>{v}, dy, g);
+      }
     } else {
-      AConvT<float> a{ConvView<float>{(const float*)X, cg, 1.f}};
-      rc = launch_grad_gemm(a, BRow{dY, F}, g, db, &db_fused);
+      rc = launch_grad_gemm(AConvT<float>{ConvView<float>{(const float*)X, cg, 1.f}}, dy, g, db, &db_fused);
     }
     if (rc) return rc;
   }
@@ -1640,45 +1497,39 @@ int b200rl_conv2d_bwd(const void* X, int x_is_u8, float x_scale, const float* Wt
     rc = colsum(dY, db, M, F, accumulate, workspace, ws_bytes, st);
     if (rc) return rc;
   }
-  if (dX && gemm_mode() != 0 && (c->C & 3) == 0 && K >= 16 && M >= 32 && F >= 8) {
-    // tcgen05 path: dY @ W^T with the col2im scatter-add fused into the epilogue
-    const int64_t total = (int64_t)c->N * c->H * c->W * c->C;
+  if (!dX) return B200RL_OK;
+  const int64_t total = (int64_t)c->N * c->H * c->W * c->C;
+  const ARow da{dY, F};
+  const BCol wt{Wt, F};
+  GemmArgs g{nullptr, nullptr, M, K, F, B200RL_ACT_NONE, 0, nullptr, 0, st};
+  if ((c->C & 3) == 0 && tensor_route(da, wt, g)) {
+    // dY @ W^T with the col2im scatter-add fused into the epilogue
     cudaError_t e = cudaMemsetAsync(dX, 0, (size_t)total * sizeof(float), st);
     if (e != cudaSuccess) {
       set_error("conv2d_bwd: memset failed: %s", cudaGetErrorString(e));
       return B200RL_ERR_CUDA;
     }
-    GemmArgs g{nullptr, nullptr, M, K, F, B200RL_ACT_NONE, 0, nullptr, 0, st};
-    tc::EpiArgs epi{cg, dX};
+    tc2::EpiArgs epi{cg, dX};
     epi.mask = mask;
-    const ARow da{dY, F};
-    const BCol db_{Wt, F};
     // neighbour pre-sum of the col2im epilogue (tc2_gemm.cuh): the partner column group sits
     // stride * C = 64 columns away, i.e. in the other half of the same 128-column tile (the Mnih
     // conv2 (k4 s2 C32) and conv3 (k3 s1 C64) input gradients); B200RL_COL2IM_MERGE=0 turns it off
     static const int merge_env = [] { const char* e = getenv("B200RL_COL2IM_MERGE"); return e ? atoi(e) : 1; }();
-    if (merge_env && (int64_t)c->stride * c->C == 64 && (c->C & 15) == 0 && cg.OW > 1) epi.merge_cols = 64;
-    if (use_tc2(da, db_, g)) {
-      if (epi.merge_cols) {
-        if (gemm_mode() == 2) rc = launch_tc2_cfg<128, 1, tc::EPI_COL2IM_MERGE>(da, db_, g, epi);
-        else rc = launch_tc2_cfg<128, 3, tc::EPI_COL2IM_MERGE>(da, db_, g, epi);
-      } else if (gemm_mode() == 2) rc = launch_tc2_cfg<128, 1, tc::EPI_COL2IM>(da, db_, g, epi);
-      else rc = launch_tc2_cfg<128, 3, tc::EPI_COL2IM>(da, db_, g, epi);
-    } else if (gemm_mode() == 2) rc = launch_tc_cfg<128, 3, 1, tc::EPI_COL2IM>(da, db_, g, epi);
-    else rc = launch_tc_cfg<128, 3, 3, tc::EPI_COL2IM>(da, db_, g, epi);
-    if (rc) return rc;
-  } else if (dX) {  // dcol[M,K] = dY @ W^T, then gather-form col2im
-    const int64_t need = M * K * (int64_t)sizeof(float);
-    B200RL_CHECK_ARG(workspace && ws_bytes >= need,
-                     "conv2d_bwd: input gradient needs %lld bytes of workspace",
-                     (long long)need);
-    GemmArgs g{(float*)workspace, nullptr, M, K, F, B200RL_ACT_NONE, 0, nullptr, 0, st};
-    rc = launch_gemm(ARow{dY, F}, BCol{Wt, F}, g);
-    if (rc) return rc;
-    const int64_t total = (int64_t)c->N * c->H * c->W * c->C;
-    B200RL_LAUNCH(col2im_kernel, (unsigned)((total + 255) / 256), 256, 0, st, (const float*)workspace, dX, cg, total, (int)K, mask);
-    B200RL_CHECK_LAUNCH("col2im");
+    if (merge_env && (int64_t)c->stride * c->C == 64 && (c->C & 15) == 0 && cg.OW > 1) {
+      epi.merge_cols = 64;
+      return launch_tensor<tc2::EPI_COL2IM_MERGE>(da, wt, g, epi);
+    }
+    return launch_tensor<tc2::EPI_COL2IM>(da, wt, g, epi);
   }
+  // dcol[M,K] = dY @ W^T, then gather-form col2im
+  const int64_t need = M * K * (int64_t)sizeof(float);
+  B200RL_CHECK_ARG(workspace && ws_bytes >= need,
+                   "conv2d_bwd: input gradient needs %lld bytes of workspace", (long long)need);
+  g.C = (float*)workspace;
+  rc = launch_gemm(da, wt, g);
+  if (rc) return rc;
+  B200RL_LAUNCH(col2im_kernel, (unsigned)((total + 255) / 256), 256, 0, st, (const float*)workspace, dX, cg, total, (int)K, mask);
+  B200RL_CHECK_LAUNCH("col2im");
   return B200RL_OK;
 }
 

@@ -1,13 +1,19 @@
-// Persistent, warp-specialised tcgen05 GEMM (second generation of tc_gemm.cuh).
+// Persistent, warp-specialised tcgen05 GEMM for the Q / actor / critic networks: tcgen05.mma
+// (kind::tf32) with TMEM accumulators, fp32-grade accuracy through the 3xTF32 split.
 //
 //   C[M,N] (+)= act(A[M,K] @ B[K,N] + bias)   over the operand views of nn.cu, 3xTF32 or 1xTF32
 //
-// What changed against tc_gemm.cuh, and why (profiles/r2/README.md, run 1): the first kernel ran
-// ONE output tile per CTA with 8 producer warps that pulled operands through registers
-// (LDG -> split -> STS); ncu showed (a) 80-225 KB of SASS per instantiation, i.e. an instruction
-// cache that never warms, (b) producers stalled on their own loads (long-scoreboard on the first
-// use of every LDG) with ~400 issued instructions per K block per warp for 6 loads, (c) the
-// prologue (TMEM allocation, barrier init) and the epilogue exposed on every tile.  Here:
+// Why 3xTF32: north_star parity is 1e-5 relative on the loss; one TF32 pass keeps ~11 mantissa
+// bits (1e-3).  Each fp32 operand x is split into hi = x with the low 13 mantissa bits cleared and
+// lo = x - hi (exact); the tensor core accumulates lo_a*hi_b + hi_a*lo_b + hi_a*hi_b into the same
+// fp32 TMEM accumulator (the dropped lo*lo term is 2^-22 relative).  Raw uint8 pixels are exact in
+// TF32, so an exact A operand needs no lo plane (a*b_lo + a*b_hi).
+//
+// History (profiles/r2/README.md, run 1): the first-generation kernel ran ONE output tile per CTA
+// with 8 producer warps that pulled operands through registers (LDG -> split -> STS); ncu showed
+// (a) 80-225 KB of SASS per instantiation, i.e. an instruction cache that never warms, (b)
+// producers stalled on their own loads, (c) the prologue (TMEM allocation, barrier init) and the
+// epilogue exposed on every tile.  Here:
 //
 //   * one CTA per SM, persistent over (split, m-tile, n-tile) work items;
 //   * warps 0-7   LOADERS: cp.async (LDGSTS, 16 B, zero-fill) of the raw operand chunks straight
@@ -24,32 +30,131 @@
 //                 K step is 2 MMAs and an exact-A (uint8) step is 1;
 //   * warps 17+   EPILOGUE of tile i (tcgen05.ld, bias/activation/act' mask, stores, split-K
 //                 red.add, fused col2im scatter-add) overlaps the main loop of tile i+1;
-//   * every loop that is not a fixed 4-8x unroll is rolled, the scalar fall-back paths live in
-//                 tc_gemm.cuh (the host dispatch only sends 16-byte-vectorisable views here).
+//   * every loop that is not a fixed 4-8x unroll is rolled.  There are no scalar paths: the host
+//                 dispatch only sends views whose every 16-byte chunk is contiguous and aligned
+//                 (tc2_ok in nn.cu); every other shape takes the FFMA kernel.
 //
-// Shared-memory operand layouts, descriptors and the 3xTF32 scheme are those of tc_gemm.cuh.
+// Descriptors follow cute/arch/mma_sm100_desc.hpp (SmemDescriptor: K-major SWIZZLE_128B,
+// SBO = 1024 B, version 1; InstrDescriptor: F32 accumulate, TF32 x TF32, M = 128, N = BN).
 #pragma once
 #include <cuda.h>
+#include <cuda_runtime.h>
+#include <stdint.h>
 
 #include <type_traits>
-
-#include "tc_gemm.cuh"
 
 namespace b200rl {
 namespace tc2 {
 
-using tc::EpiArgs;
-using tc::EPI_ATOMIC;
-using tc::EPI_COL2IM;
-using tc::EPI_COL2IM_MERGE;
-using tc::EPI_STORE;
-using tc::kBK;
-using tc::kBM;
-using tc::mbar_arrive;
-using tc::mbar_init;
-using tc::mbar_wait;
-using tc::smem_addr;
+// ---- tcgen05 / mbarrier primitives, shared-memory layouts ---------------------------------------
+constexpr int kBM = 128;
+constexpr int kBK = 32;                    // fp32 elements = 128 bytes = one swizzle row
 
+__device__ __forceinline__ uint32_t smem_addr(const void* p) {
+  return (uint32_t)__cvta_generic_to_shared(p);
+}
+__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
+  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+// Spin on the non-blocking test_wait (the `poll` A/B switch, bit 6 of g_tc2_flags; the default
+// is the suspending try_wait of mbar_wait_hw below).
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+  uint32_t done;
+  do {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+        "selp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(done)
+        : "r"(bar), "r"(parity)
+        : "memory");
+  } while (!done);
+}
+__device__ __forceinline__ void tc_commit(uint32_t bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar)
+               : "memory");
+}
+__device__ __forceinline__ void tc_mma_tf32(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc,
+                                            uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+
+// K-major, SWIZZLE_128B, 8-row groups 1024 B apart (cute SmemDescriptor, version 1).
+__device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
+  uint64_t d = 0;
+  d |= (uint64_t)((saddr >> 4) & 0x3FFF);          // start address
+  d |= (uint64_t)1 << 16;                          // leading byte offset (unused for SW128 K-major)
+  d |= (uint64_t)(1024 >> 4) << 32;                // stride byte offset
+  d |= (uint64_t)1 << 46;                          // version = 1 (sm_100)
+  d |= (uint64_t)2 << 61;                          // layout type SWIZZLE_128B
+  return d;
+}
+// MN-major tf32 operands: SWIZZLE_128B_BASE32B is the only layout the tensor core accepts for
+// 32-bit MN-major data (cutlass sm100_common.inl: "for mn-major tf32 operands, SW128_32B is the
+// only available smem layout"; cute Layout_MN_SW128_32B_Atom = Swizzle<2,5,2> o (1024 bit, 4) :
+// (1, 1024 bit)).  A k-row holds 32 consecutive M/N elements (128 B); 4 k-rows form a 512 B atom
+// in which the 32-byte blocks of a row are XORed with the row index; LBO = distance between
+// 32-element M/N groups, SBO = distance between 4-row k atoms (one K=8 MMA spans two atoms).
+__device__ __forceinline__ uint64_t make_desc_mn(uint32_t saddr, uint32_t sbo_bytes) {
+  uint64_t d = 0;
+  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
+  d |= (uint64_t)(512 >> 4) << 16;                 // LBO: next 32-row M/N group (adjacent atom)
+  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;  // SBO: next 4-row k atom = (ROWS/32) atoms
+  d |= (uint64_t)1 << 46;                          // version = 1 (sm_100)
+  d |= (uint64_t)1 << 61;                          // layout type 1 = SWIZZLE_128B_BASE32B
+  return d;
+}
+__host__ __device__ constexpr uint32_t make_idesc(int bn, bool a_mn, bool b_mn) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
+         ((uint32_t)(bn >> 3) << 17) | ((uint32_t)(kBM >> 4) << 24);
+}
+// byte offset of the 16-byte chunk holding rows 4*cm..4*cm+3 at reduction index k (0..31) in an
+// MN-major tile: 512 B atoms (32 rows x 4 k) tiled M/N-fastest (the arrangement cute's
+// tile_to_shape produces), rows 128 B apart; inside a row the 32-byte block index is XORed with
+// (k & 3).
+template <int ROWS>
+__device__ __forceinline__ uint32_t mn128(uint32_t cm, uint32_t k) {
+  const uint32_t c = cm & 7u, kin = k & 3u;
+  const uint32_t blk = (((c >> 1) ^ kin) << 1) | (c & 1u);   // 32-byte block XOR k, 16 B half kept
+  return ((k >> 2) * (ROWS / 32) + (cm >> 3)) * 512u + kin * 128u + (blk << 4);
+}
+// byte offset of 16-byte chunk j (0..7) of row r inside a K-major [rows x 128 B] SWIZZLE_128B tile
+__device__ __forceinline__ uint32_t sw128(uint32_t r, uint32_t j) {
+  return (r >> 3) * 1024u + (r & 7u) * 128u + ((j ^ (r & 7u)) << 4);
+}
+
+// Epilogue variants.  EPI_STORE: C (+)= act(acc + bias) or split-K partial.  EPI_ATOMIC: C += acc
+// with red.global.add (split-K without a reduce pass; C pre-zeroed).  EPI_COL2IM: the GEMM is
+// dcol[pos, (ky,kx,c)] = dY @ W^T of a convolution input gradient and every 4-channel group is
+// scatter-added straight into dX[n, oy*s+ky, ox*s+kx, c..c+3] with one red.global.add.v4.f32 --
+// the [M, KH*KW*C] dcol matrix is never materialised and split-K partials need no reduction pass
+// (dX must be zeroed by the caller; summation order of the <= KH*KW/s^2 contributions per element
+// is not fixed).  EPI_COL2IM_MERGE: EPI_COL2IM with the neighbour pre-sum of EpiArgs::merge_cols
+// (its own instantiation, so that neither variant pays for the other's registers).
+constexpr int EPI_STORE = 0;
+constexpr int EPI_COL2IM = 1;
+constexpr int EPI_ATOMIC = 2;
+constexpr int EPI_COL2IM_MERGE = 3;
+struct EpiArgs {
+  ConvGeom g;
+  float* dx;
+  ActMask mask;     // EPI_STORE / EPI_COL2IM: multiply the input gradient by act'(mask.y)
+  float* colsum;    // EPI_ATOMIC with an MN-major B view: column sums of B (bias gradient) += here
+  // EPI_COL2IM_MERGE: columns c and c + merge_cols (= stride * C) of NEIGHBOURING output positions
+  // (ox + 1, ox) address the same input element; the epilogue adds them with a lane shuffle before
+  // the red.global.add.  0: every column group is scattered.
+  int merge_cols;
+};
+
+// ---- the persistent kernel ----------------------------------------------------------------------
 // Run-7 trace: once the MMA count per K step dropped (WIDE below), the K-block period (620-720 ns)
 // stayed above every role's busy time (loaders ~400-500, converters ~350-450, MMA issue ~230-410):
 // a loader and a converter warp share each scheduler and both are chains of dependent scalar
@@ -253,7 +358,7 @@ struct LoadKContigF32 {
                                              int64_t delta) {
     j = t & 7;
     const int r0 = t >> 3;
-    dst0 = tc::sw128((uint32_t)r0, (uint32_t)j);
+    dst0 = sw128((uint32_t)r0, (uint32_t)j);
     ok = 0;
 #pragma unroll
     for (int i = 0; i < NR; ++i) {
@@ -295,7 +400,7 @@ struct LoadMnF32 {                                 // LROWS: rows of the shared-
     ok = r < row_limit;                            // rows % 4 == 0 (host check)
     rowp = reinterpret_cast<const char*>(v.addr(ok ? v.row_off(r) : 0)) + delta;
 #pragma unroll
-    for (int i = 0; i < NC; ++i) dst[i] = tc::mn128<LROWS>((uint32_t)cm, (uint32_t)(kk0 + KSTEP * i));
+    for (int i = 0; i < NC; ++i) dst[i] = mn128<LROWS>((uint32_t)cm, (uint32_t)(kk0 + KSTEP * i));
   }
   __device__ __forceinline__ void issue(const V& v, uint32_t plane, int64_t k0, int64_t ke) {
     if constexpr (V::kLinearK) {
@@ -467,7 +572,7 @@ __device__ __forceinline__ void convert_u8_kcontig(uint32_t raw, uint32_t plane,
   for (int q = 0; q < 4; ++q) {
     float4 o;
     u8x4_to_f32(w[q], o);
-    sts128(plane + tc::sw128(row, 4u * h + (uint32_t)q), o);
+    sts128(plane + sw128(row, 4u * h + (uint32_t)q), o);
   }
 }
 // raw [32 k][128 B] uint8 -> MN-major fp32 tile (128 rows).  Chunk (kk, c) = the 16 patch
@@ -493,7 +598,7 @@ __device__ __forceinline__ void convert_u8_mn(uint32_t raw, uint32_t plane, int 
     for (int q = 0; q < 4; ++q) {
       float4 o;
       u8x4_to_f32(w[q], o);
-      sts128(plane + tc::mn128<kBM>(4u * c + ((uint32_t)q ^ cb), kk), o);
+      sts128(plane + mn128<kBM>(4u * c + ((uint32_t)q ^ cb), kk), o);
     }
   }
 }
@@ -690,8 +795,8 @@ __global__ void __launch_bounds__(kThreads, 1)
   } else if (warp == kMmaWarp) {
     // ======================= MMA issuer =======================
     if (lane == 0) {
-      constexpr uint32_t idesc = tc::make_idesc(BN, !AL::kKContig, !BL::kKContig);
-      constexpr uint32_t idesc_w = tc::make_idesc(2 * BN, !AL::kKContig, !BL::kKContig);
+      constexpr uint32_t idesc = make_idesc(BN, !AL::kKContig, !BL::kKContig);
+      constexpr uint32_t idesc_w = make_idesc(2 * BN, !AL::kKContig, !BL::kKContig);
       constexpr int kBRows = kWide ? 2 * BN : BN;   // rows of the MN-major B tile layout
       // One thread issues every MMA, so its scalar instruction stream IS the K-loop rate once the
       // operands arrive (run 4 trace: 560 ns per K block, ~30 instructions per MMA, most of them
@@ -701,8 +806,8 @@ __global__ void __launch_bounds__(kThreads, 1)
       constexpr uint32_t kaStep = AL::kKContig ? 2u : (2u * (kBM / 32) * 512u) >> 4;   // per K = 8
       constexpr uint32_t kbStep = BL::kKContig ? 2u : (2u * (kBRows / 32) * 512u) >> 4;
       constexpr uint32_t kStageStep = (uint32_t)L::kStage >> 4;
-      const uint64_t dA = AL::kKContig ? tc::make_desc(0) : tc::make_desc_mn(0, (kBM / 32) * 512u);
-      const uint64_t dB = BL::kKContig ? tc::make_desc(0) : tc::make_desc_mn(0, (kBRows / 32) * 512u);
+      const uint64_t dA = AL::kKContig ? make_desc(0) : make_desc_mn(0, (kBM / 32) * 512u);
+      const uint64_t dB = BL::kKContig ? make_desc(0) : make_desc_mn(0, (kBRows / 32) * 512u);
       const uint32_t fa_hi = smem_base >> 4, fa_lo = (smem_base + L::kATile) >> 4;
       const uint32_t fb_hi = (smem_base + kOffB) >> 4, fb_lo = (smem_base + kOffB + L::kBTile) >> 4;
       const bool no_mma = (g_tc2_flags & 32) != 0;
@@ -731,26 +836,26 @@ __global__ void __launch_bounds__(kThreads, 1)
             const uint32_t oa = so + (uint32_t)ks * kaStep, ob = so + (uint32_t)ks * kbStep;
             const uint32_t acc0 = ks == 0 ? first : 1u;
             if (kWide && AL::kExact) {
-              tc::tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc_w, acc0);
+              tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc_w, acc0);
             } else if (kWide) {
               // columns [0, BN): A_hi B_hi + A_lo B_hi; columns [BN, 2 BN): A_hi B_lo
-              tc::tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc_w, acc0);
-              tc::tc_mma_tf32(tmem_d, dA + (fa_lo + oa), dB + (fb_hi + ob), idesc, 1u);
+              tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc_w, acc0);
+              tc_mma_tf32(tmem_d, dA + (fa_lo + oa), dB + (fb_hi + ob), idesc, 1u);
             } else if (PASSES == 3 && AL::kExact) {
-              tc::tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_lo + ob), idesc, acc0);
-              tc::tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc, 1u);
+              tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_lo + ob), idesc, acc0);
+              tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc, 1u);
             } else if (PASSES == 3) {
-              tc::tc_mma_tf32(tmem_d, dA + (fa_lo + oa), dB + (fb_hi + ob), idesc, acc0);
-              tc::tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_lo + ob), idesc, 1u);
-              tc::tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc, 1u);
+              tc_mma_tf32(tmem_d, dA + (fa_lo + oa), dB + (fb_hi + ob), idesc, acc0);
+              tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_lo + ob), idesc, 1u);
+              tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc, 1u);
             } else {
-              tc::tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc, acc0);
+              tc_mma_tf32(tmem_d, dA + (fa_hi + oa), dB + (fb_hi + ob), idesc, acc0);
             }
           }
-          tc::tc_commit(smem_addr(&empty[s]));
+          tc_commit(smem_addr(&empty[s]));
           trace(tr, 2, it, 1);
         }
-        tc::tc_commit(smem_addr(&acc_full[buf]));
+        tc_commit(smem_addr(&acc_full[buf]));
       }
     }
     __syncwarp();

@@ -343,19 +343,20 @@ int b200rl_concat2(const float* a, int64_t lda, int64_t da, const float* b, int6
 /* GEMM engine for every dense / conv entry point below: 0 = fp32 FFMA register-tiled kernel,
  * 1 = tcgen05 tensor cores with the 3xTF32 split (fp32-grade accuracy, TMEM accumulators),
  * 2 = tcgen05 single-pass TF32 (~1e-3 relative; NOT within the 1e-5 parity bar).
- * Default: env B200RL_GEMM_MODE, else 1.  Outputs narrower than 16 columns (Q head, value head)
- * always use mode 0. */
+ * Default: env B200RL_GEMM_MODE, else 1.  In modes 1 and 2 a GEMM takes the tensor cores when
+ * N >= 16, M >= 32, K >= 8 and both operands can be read as aligned 16-byte chunks (reduction
+ * length and leading dimensions multiples of 4, 16-byte aligned bases; uint8 conv inputs with
+ * KW*C, stride*C, W*C and the image stride multiples of 16); every other GEMM runs on the FFMA
+ * kernel.  Heads of <= 16 outputs and inputs of <= 32 features have kernels of their own in
+ * modes 1 and 2. */
 int b200rl_set_gemm_mode(int mode);
-/* Profiling aid: device buffer of int64[64][8] that receives %globaltimer phase stamps of the
- * first 64 CTAs of every tcgen05 GEMM launch (NULL disables). */
-int b200rl_tc_debug_buffer(long long* dev_buf);
-/* Profiling/bring-up aid: selects an MN-major tile layout experiment (0 = production). */
-int b200rl_tc_debug_variant(int v);
-/* Second-generation GEMM kernel (tc2_gemm.cuh) switches.  bit 0: store an explicitly masked
- * TF32 "hi" plane instead of using the raw fp32 operand tile for it (the tensor core ignores the
- * low 13 mantissa bits; both settings are bit-identical, the default saves the store).  bit 1 (or B200RL_TC2=0 in the environment): route every GEMM to the
- * first-generation kernel (A/B comparisons in profiles/tc2_check.py).  bit 2: load plain 2-D
- * operands with cp.async like the im2col views instead of TMA tensor tiles. */
+/* Tensor-core GEMM kernel (tc2_gemm.cuh) switches.  bit 0: store an explicitly masked TF32 "hi"
+ * plane instead of using the raw fp32 operand tile for it (the tensor core ignores the low 13
+ * mantissa bits; both settings are bit-identical, the default saves the store).  bit 1: unused.
+ * bit 2: load plain 2-D operands with cp.async like the im2col views instead of TMA tensor
+ * tiles.  bits 3-5: timing ablations (profiles/tc2_ablate.py; results are garbage).  bit 6: poll
+ * mbarriers with test_wait instead of try_wait.  B200RL_TC2_FLAGS in the environment sets the
+ * initial value. */
 int b200rl_set_tc2_flags(int flags);
 /* Work distribution of the persistent tcgen05 GEMM: 0 (default) static striding over the CTAs,
  * 1 dynamic (global tile counter) -- set by the data-parallel Learner (train/learner.py:104-143 in

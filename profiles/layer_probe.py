@@ -1,9 +1,9 @@
 """Per-layer GEMM timing of the Mnih'15 Q-network at batch 256 (config 2 shapes): forward, input
 gradient (dX) and parameter gradient (dW + db) of every layer, each timed as R back-to-back
 launches replayed from one CUDA graph (CUDA events on the launch stream; the number is kernel
-time, not Python launch overhead), plus the %globaltimer phase stamps of the tcgen05 kernel.
+time, not Python launch overhead).
 
-    python profiles/layer_probe.py [--reps 20] [--batch 256] [--stamps]
+    python profiles/layer_probe.py [--reps 20] [--batch 256]
 
 Prints one JSON line per (layer, pass).  `gflop` is the fp32-equivalent work of the GEMM,
 `tflops` = gflop / time.  Used by profiles/README.md's per-layer table.
@@ -13,7 +13,6 @@ import json
 import os
 import sys
 
-import numpy as np
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -21,10 +20,6 @@ from agents_b200 import _lib  # noqa: E402
 from agents_b200.networks import layers as L  # noqa: E402
 from agents_b200.networks import q_network  # noqa: E402
 from agents_b200.specs import tensor_spec  # noqa: E402
-
-NAMES = ['start', 'alloc_sync', 'producers_done', 'mma_issued', 'accum_ready', 'epilogue_done',
-         'dealloc']
-
 
 def timed_graph(fn, reps, iters=5):
   """Captures `reps` calls of fn into one graph, replays it `iters` times; returns us per call."""
@@ -49,29 +44,10 @@ def timed_graph(fn, reps, iters=5):
   return best
 
 
-def stamps(fn, dbg):
-  dbg.zero_()
-  torch.cuda.synchronize()
-  _lib.call('b200rl_tc_debug_buffer', _lib.ptr(dbg))
-  fn()
-  torch.cuda.synchronize()
-  _lib.call('b200rl_tc_debug_buffer', None)
-  d = dbg.view(64, 8).cpu().numpy()
-  valid = d[:, 6] > 0
-  if not valid.any():
-    return None
-  dd = d[valid, 1:7] - d[valid, :1]
-  med = np.median(dd, axis=0)
-  return dict(phases_ns={NAMES[i + 1]: int(med[i]) for i in range(6)},
-              start_spread_ns=int(d[valid, 0].max() - d[valid, 0].min()),
-              span_ns=int(d[valid, 6].max() - d[valid, 0].min()), ctas_seen=int(valid.sum()))
-
-
 def main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--reps', type=int, default=20)
   ap.add_argument('--batch', type=int, default=256)
-  ap.add_argument('--stamps', action='store_true')
   args = ap.parse_args()
   dev = torch.device('cuda:0')
   obs_spec = tensor_spec.TensorSpec((84, 84, 4), torch.uint8)
@@ -83,7 +59,6 @@ def main():
   B = args.batch
   x = torch.randint(0, 256, (B, 84, 84, 4), dtype=torch.uint8, device=dev)
   layers = [l for l in net.layers if not isinstance(l, L.CastScale)]
-  dbg = torch.zeros(64 * 8, dtype=torch.int64, device=dev)
   acts, h = [], x
   for l in layers:
     y = l.forward(h)
@@ -113,10 +88,6 @@ def main():
       us = timed_graph(fn, args.reps)
       line = dict(layer=name, op=pname, M=m, N=n, K=k, us=round(us, 2), gflop=round(gflop, 3),
                   tflops=round(gflop / us * 1e-3 * 1e6 / 1e3, 2))
-      if args.stamps:
-        st = stamps(fn, dbg)
-        if st:
-          line.update(st)
       print(json.dumps(line), flush=True)
     prev_act = l._act
   # separate kernels that the fused paths replace / that remain on the step

@@ -2,7 +2,7 @@
 cudaProfilerStop, after two warm-up passes -- the target of the ncu captures:
 
     ncu --set full --clock-control none --import-source on --profile-from-start off \
-        -k regex:tc_gemm -o gpurun_out/r2_net python profiles/net_once.py
+        -k regex:tc2_gemm -o net_once_report python profiles/net_once.py
 """
 import os
 import sys

@@ -1,4 +1,4 @@
-"""tc2 (persistent cp.async tcgen05 GEMM) against the first-generation kernel, layer by layer:
+"""tc2 (persistent cp.async tcgen05 GEMM) against the fp32 FFMA engine (gemm mode 0), layer by layer:
 max relative difference and time of forward / dX / dW for the Mnih'15 layers (batch 256), the
 PPO (200,100) tanh MLP at 4096x128 rows and the SAC (256,256) critic at batch 1024.
 A progress line is flushed BEFORE every launch, so a hang names its culprit.
@@ -22,6 +22,7 @@ ap.add_argument('--flags', type=int, default=0)
 ap.add_argument('--only', default='')
 args = ap.parse_args()
 dev = torch.device('cuda:0')
+_lib.call('b200rl_set_tc2_flags', args.flags)
 gen = torch.Generator(device=dev).manual_seed(0)
 
 
@@ -63,16 +64,16 @@ def run_both(name, op, fn, outs):
   if args.only and args.only not in f'{name}.{op}':
     return
   res = {}
-  for tag, flags in (('tc1', 2), ('tc2', args.flags)):
+  for tag, mode in (('ffma', 0), ('tc2', 1)):
     say(progress=f'{name}.{op}.{tag}')
-    _lib.call('b200rl_set_tc2_flags', flags)
+    _lib.call('b200rl_set_gemm_mode', mode)
     o = fn()
     torch.cuda.synchronize()
     res[tag] = [t.clone() for t in o]
     res[tag + '_us'] = timed(fn, args.reps)
-  diffs = [rel(x, y) for x, y in zip(res['tc2'], res['tc1'])]
-  say(layer=name, op=op, tc1_us=round(res['tc1_us'], 2), tc2_us=round(res['tc2_us'], 2),
-      speedup=round(res['tc1_us'] / res['tc2_us'], 2), max_rel_diff=max(diffs), outs=outs)
+  diffs = [rel(x, y) for x, y in zip(res['tc2'], res['ffma'])]
+  say(layer=name, op=op, ffma_us=round(res['ffma_us'], 2), tc2_us=round(res['tc2_us'], 2),
+      speedup=round(res['ffma_us'] / res['tc2_us'], 2), max_rel_diff=max(diffs), outs=outs)
 
 
 def check_layer(name, layer, x, prev_act):
@@ -103,11 +104,12 @@ h = check_layer('fc1', L.Dense(512, activation='relu'), h, 1)
 # odd sizes: ragged M / N tiles, K not a multiple of 32
 xr = torch.randn(1000, 200, device=dev, generator=gen)
 check_layer('ragged_1000x200x100', L.Dense(100, activation='tanh'), xr, 2)
-# PPO MLP (4096 x 128 rows; the 17-wide input layer stays on the FFMA path)
+# PPO MLP (4096 x 128 rows; the 17-wide input layer has kernels of its own)
 xp = torch.randn(4096 * 128, 200, device=dev, generator=gen).tanh()
 check_layer('ppo_200x100', L.Dense(100, activation='tanh'), xp, 2)
 # SAC critic
 xs = torch.randn(1024, 256, device=dev, generator=gen).relu()
 check_layer('sac_256x256', L.Dense(256, activation='relu'), xs, 1)
 _lib.call('b200rl_set_tc2_flags', 0)
+_lib.call('b200rl_set_gemm_mode', 1)
 say(done=True)

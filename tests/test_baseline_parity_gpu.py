@@ -123,13 +123,15 @@ def test_config2_dqn_mnih_batch256_train_parity(cuda):
 
 def test_dqn_train_parity_all_layers_on_tensor_cores(cuda):
   """5 steps of a conv net whose every layer has >= 16 output channels at batch 32, so conv1 also
-  takes the tcgen05 path (numpy oracle, Adam, n-step 2, clipping, Polyak)."""
+  takes the tcgen05 path (numpy oracle, Adam, n-step 2, clipping, Polyak).  conv1 is k4 s4 on the
+  28x28x4 uint8 input: stride * C = 16, so the raw-pixel loader of the tensor-core kernel can copy
+  its patches in 16-byte chunks (tests/test_gemm_route_gpu.py pins the route)."""
   rng = np.random.RandomState(3)
   A, B, n = 4, 32, 2
   obs_spec = tensor_spec.TensorSpec((28, 28, 4), torch.uint8)
   act_spec = tensor_spec.BoundedTensorSpec((), torch.int32, 0, A - 1)
   net = q_network.QNetwork(obs_spec, act_spec, preprocessing_layers=L.CastScale(255.),
-                           conv_layer_params=((16, 4, 2), (32, 3, 1)), fc_layer_params=(64,),
+                           conv_layer_params=((16, 4, 4), (32, 3, 1)), fc_layer_params=(64,),
                            device=cuda).set_seed(1)
   agent = dqn_agent.DdqnAgent(ts.time_step_spec(obs_spec), act_spec, q_network=net,
                               optimizer=optimizers.AdamOptimizer(1e-3), n_step_update=n,
